@@ -21,6 +21,8 @@ config.batched   = BASELINE config 4 (1024 goals, 1M-vertex terrain, goal k -> r
                    plans/s, HBM fraction and 8 sampled fields against the oracle -- inside `config` because the driver
                    keeps that object for every N.
 --impl reference: the oracle on the host cores, one independent plan per thread.
+--dump-outputs DIR: the arrays the last timed plan returned, as DIR/<name>.npy (dump_outputs()); the inputs are seeded, so
+                   two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -36,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 CVP_BYTES_PER_VERTEX = 208       # SURVEY.md 8d
 METRIC = "vertex-relaxations/sec"
@@ -133,6 +136,21 @@ def parity_block(got_dist, got_pred, ref, got_cut=None):
     return out
 
 
+DUMP_MAX_VERTICES = 1 << 20     # 32 B per dumped vertex (two f32, three f64 arrays): at most 32 MiB in all
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the per-vertex arrays a caller of the timed plan receives (potential, predecessor, direction, cutting
+    face), so that two builds can be compared output for output.  Above DUMP_MAX_VERTICES vertices a fixed, seeded sample
+    of vertices is written; vertex_index.npy names them.  Float arrays stay float32, index arrays become float64 (exact)."""
+    V = next(iter(arrays.values())).size
+    idx = np.arange(V) if V <= DUMP_MAX_VERTICES else np.sort(np.random.default_rng(0).choice(V, DUMP_MAX_VERTICES, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "vertex_index.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[idx].astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 CONFIG_KEYS = ("workload", "vertices", "faces", "edges", "plans_per_step_per_gpu", "sharding", "l2", "parity", "config3", "batched")
 
 
@@ -225,7 +243,11 @@ def main():
     ap.add_argument("--no-config3", action="store_true")
     ap.add_argument("--no-other-kernels", action="store_true")
     ap.add_argument("--submesh-from", type=int, default=3000, help="grid side from which the 1M sub-mesh parity spot check runs (config 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed plan returned (rank 0) to DIR/<name>.npy, see dump_outputs()")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -296,10 +318,13 @@ def main():
         dt_max = dt; total_settled = float(settled)
     clocks = sampler.stop(local)
     value = total_settled * args.steps / dt_max
-    # the result of the LAST TIMED plan, for the parity block (rank 0)
+    # the result of the LAST TIMED plan, for the parity block and the output dump (rank 0)
     h_timed = None
-    if rank == 0 and not args.no_cpu_baseline:
+    if rank == 0 and (not args.no_cpu_baseline or args.dump_outputs):
         h_timed = {"dist": d_dist.cpu().numpy(), "pred": d_pred.cpu().numpy().view(np.uint32), "cut": d_cut.cpu().numpy()}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"dist": h_timed["dist"], "pred": h_timed["pred"], "direction": d_dir.cpu().numpy(),
+                                             "cutting_face": h_timed["cut"]})
 
     # ---- e2e: host buffers through the C ABI, copies inside the timed region ----
     from mesh_navigation_b200.api import CVPMeshPlanner

@@ -6,9 +6,12 @@ reference legs may import this module.  The product package
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -28,12 +31,13 @@ _lib = None
 
 def use_native_build() -> str:
     """CPU-baseline legs of bench.py only: rebuild the oracle ON THIS HOST with `-O3 -march=native -DNDEBUG` (BASELINE.md
-    section 2) into oracle/_native/ and route every later call there.  The default liboracle.so is generic x86-64 because it
-    is built in the build container and travels to the GPU box; -ffp-contract=off is kept, so results do not change.
+    section 2) into a temporary directory (the source tree may be read-only), removed at exit, and route every later call
+    there.  The default liboracle.so is generic x86-64 because it may be built on another host than the one that runs it;
+    -ffp-contract=off is kept, so results do not change.
     Returns the flag string actually in effect (the generic build if the native one cannot be compiled)."""
     global _SO, _lib
-    out_dir = os.path.join(_HERE, "_native")
-    os.makedirs(out_dir, exist_ok=True)
+    out_dir = tempfile.mkdtemp(prefix="oracle_native_")
+    atexit.register(shutil.rmtree, out_dir, ignore_errors=True)
     so = os.path.join(out_dir, "liboracle_native.so")
     flags = ["-O3", "-march=native", "-DNDEBUG", "-ffp-contract=off", "-fPIC", "-std=c++17"]
     try:

@@ -89,12 +89,17 @@ def test_cpp_host_mirror_on_the_cpu_interpreter(emu_lib, tmp_path, oracle_mod):
     assert "cpp host mirror ok" in out.stdout
 
 
-def test_bench_orchestration_on_the_cpu_interpreter(emu_lib):
+def test_bench_orchestration_on_the_cpu_interpreter(emu_lib, tmp_path, oracle_mod):
     """bench.py's B200 arm, every leg, executed end to end on the interpreter at toy sizes (tests/emu/run_bench_on_emu.py):
-    the JSON line must carry the contract's keys and no secondary leg may have fallen into its error branch"""
+    the JSON line must carry every key of the result line and no secondary leg may have fallen into its error branch; the arrays
+    --dump-outputs writes must be the timed plan's, i.e. the oracle's plan of the same seeded input"""
     import json
+    import runpy
+
+    import numpy as np
+    dump = tmp_path / "dump"
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "emu", "run_bench_on_emu.py"), "--size", "90", "--batch-size", "50",
-                        "--batch-goals", "4", "--batch-steps", "1", "--steps", "1", "--warmup", "1"],
+                        "--batch-goals", "4", "--batch-steps", "1", "--steps", "1", "--warmup", "1", "--dump-outputs", str(dump)],
                        cwd=ROOT, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, (r.stdout + r.stderr)[-3000:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
@@ -114,6 +119,18 @@ def test_bench_orchestration_on_the_cpu_interpreter(emu_lib):
     assert line["config"]["parity"]["ok"] and line["config"]["parity"]["n_mismatch"] == 0
     assert line["config"]["config3"]["parity"]["ok"] and line["config"]["batched"]["parity_sampled"]["ok"]
     assert "parity_failed" not in line
+    got = {k: np.load(dump / f"{k}.npy") for k in ("vertex_index", "dist", "pred", "direction", "cutting_face")}
+    assert sum(os.path.getsize(dump / f"{k}.npy") for k in got) <= 64 << 20
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    B = runpy.run_path(os.path.join(ROOT, "bench.py"))
+    pos, faces = B["build_workload"](90)
+    ref = oracle_mod.OracleMesh(pos, faces)
+    ref = ref.cvp(ref.edge_distances(), np.zeros(ref.V, np.float32), *B["goal_for_rank"](pos, faces, 90, 0))
+    idx = got["vertex_index"].astype(np.int64)
+    assert np.array_equal(idx, np.arange(ref["dist"].size))
+    assert (got["dist"].view(np.uint32) == ref["dist"][idx].view(np.uint32)).all()
+    assert (got["pred"] == ref["pred"][idx]).all() and (got["cutting_face"] == ref["cutting_face"][idx]).all()
+    assert np.array_equal(got["direction"], ref["direction"][idx], equal_nan=True)
 
 
 def test_smoke_entry_on_the_cpu_interpreter(emu_lib):

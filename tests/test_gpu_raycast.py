@@ -173,12 +173,11 @@ def test_obstacle_update_with_device_resident_arrays(api, oracle_mod):
     ax = np.float32([0, 0, -1])
     mask = np.zeros(om.V, np.uint8)
     ref_le, ref_ch = om.obstacle_update(pts, T, ax, 3.0, 0.9, mask)
-    try:
-        import torch
-        on_gpu = torch.cuda.is_available()
-    except Exception:
-        on_gpu = False
+    # the loaded library decides, not torch: the CPU interpreter of the kernels (tests/emu, the only build that exports
+    # mnb_emu_switch) dereferences "device" pointers on the host, also on a machine that has a GPU
+    on_gpu = not hasattr(mm.L, "mnb_emu_switch")
     if on_gpu:      # a real device: torch owns the buffers
+        import torch
         d_pts = torch.from_numpy(pts).cuda(); d_le = torch.empty(om.V, dtype=torch.int32, device="cuda"); d_ch = torch.empty(om.V, dtype=torch.int32, device="cuda")
         ptr = lambda t: C.c_void_p(t.data_ptr()); back = lambda t, n: t[:n].cpu().numpy().view(np.uint32)
     else:           # the CPU interpreter of the kernels: "device" memory is host memory
