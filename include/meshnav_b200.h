@@ -110,6 +110,15 @@ int32_t mnb_cvp(mnb_ctx* ctx, uint32_t seed_face, const float seed_pos[3], int64
 int32_t mnb_cvp_batch(mnb_ctx* ctx, uint32_t n, const uint32_t* seed_faces /* n, host */,
                       const float* seed_pos /* 3n, host */, double cost_limit, float* out_dist);
 
+/* Batched full-field Dijkstra: n independent DijkstraMeshPlanner::dijkstra runs (robot_vertex = -1) on the installed map,
+ * one goal per thread block (or cluster), all SMs busy.  Row k of out_dist / out_pred is bit for bit what
+ * mnb_dijkstra(ctx, seed_vertices[k], -1, cost_limit, ...) writes.  out_dist [n][V] (+inf = unreached), out_pred [n][V]
+ * or NULL (self = none).  Edge weights must be >= 0.  Duplicate seeds are allowed; an invalid seed is still expanded.
+ * MNB_INVALID_START (nothing written) if a seed is >= V.  Leaves the result of the last mnb_cvp (mnb_cvp_backtrack,
+ * mnb_vector_map(pred = NULL)) untouched. */
+int32_t mnb_dijkstra_batch(mnb_ctx* ctx, uint32_t n, const uint32_t* seed_vertices /* n, host */, double cost_limit,
+                           float* out_dist, uint32_t* out_pred);
+
 /* ---- InflationLayer::waveCostInflation (inflation_layer.cpp:341-491) -----
  * lethals[n] (any order, duplicates allowed).  Uses edge_distances (:383), not edge_weights.
  * out_dist[V]: distances_ (+inf = not in the sparse map); out_cost[V]: riskiness_ =
@@ -309,6 +318,15 @@ int32_t mnb_cvp_batch_sharded(mnb_group* group, uint32_t n, const uint32_t* seed
 uint32_t mnb_group_row(mnb_group* group, uint32_t goal);
 float* mnb_group_fields(mnb_group* group, int32_t rank /* device pointer on that rank's device */);
 int32_t mnb_group_read_fields(mnb_group* group, int32_t rank, uint32_t first_goal, uint32_t count, float* out_host /* count*V */);
+/* n full-field Dijkstra plans (mnb_dijkstra_batch), sharded and gathered as mnb_cvp_batch_sharded: the distances go to the
+ * same buffers in the same layout (mnb_group_row / mnb_group_fields / mnb_group_read_fields).  With want_pred != 0 the
+ * predecessors go to a second group-owned buffer, uint32[N][pad][V] in the same layout, gathered together with the
+ * distances in one NCCL group call.  seed array: HOST. */
+int32_t mnb_dijkstra_batch_sharded(mnb_group* group, uint32_t n, const uint32_t* seed_vertices, double cost_limit,
+                                   int32_t want_pred, int32_t gather);
+uint32_t* mnb_group_preds(mnb_group* group, int32_t rank /* device pointer on that rank's device */);
+/* MNB_E_STATE unless the last sharded call was mnb_dijkstra_batch_sharded with want_pred */
+int32_t mnb_group_read_preds(mnb_group* group, int32_t rank, uint32_t first_goal, uint32_t count, uint32_t* out_host /* count*V */);
 
 #ifdef __cplusplus
 }

@@ -51,13 +51,14 @@ class Stats(C.Structure):
 EXPORTS = [
     "mnb_create", "mnb_destroy", "mnb_last_error", "mnb_set_pointer_mode", "mnb_stream", "mnb_set_mesh",
     "mnb_num_vertices", "mnb_num_faces", "mnb_num_edges", "mnb_get_edges", "mnb_get_edge_distances",
-    "mnb_compute_edge_weights", "mnb_set_costs", "mnb_dijkstra", "mnb_cvp", "mnb_cvp_batch", "mnb_inflate",
+    "mnb_compute_edge_weights", "mnb_set_costs", "mnb_dijkstra", "mnb_dijkstra_batch", "mnb_cvp", "mnb_cvp_batch", "mnb_inflate",
     "mnb_cancel", "mnb_get_stats", "mnb_set_tuning", "mnb_compute_layers", "mnb_get_vertex_normals", "mnb_vector_map", "mnb_cvp_backtrack", "mnb_locate",
     "mnb_update_vertex_costs", "mnb_get_costs", "mnb_max_combination_update", "mnb_avg_combination_update", "mnb_inflation_update",
     "mnb_inflation_vector_map", "mnb_inflation_vector_at", "mnb_set_repulsive_field",
     "mnb_cast_rays", "mnb_obstacle_update", "mnb_obstacle_reset", "mnb_normal_clearance",
     "mnb_group_create", "mnb_group_destroy", "mnb_group_size", "mnb_group_ctx", "mnb_group_last_error", "mnb_group_set_mesh",
     "mnb_group_set_costs", "mnb_group_update_vertex_costs", "mnb_cvp_batch_sharded", "mnb_group_row", "mnb_group_fields", "mnb_group_read_fields",
+    "mnb_dijkstra_batch_sharded", "mnb_group_preds", "mnb_group_read_preds",
 ]
 
 _lib = None
@@ -85,6 +86,7 @@ def load():
     L.mnb_compute_edge_weights.restype = i32; L.mnb_compute_edge_weights.argtypes = [vp, vp, dbl, vp]
     L.mnb_set_costs.restype = i32; L.mnb_set_costs.argtypes = [vp, vp, vp, vp]
     L.mnb_dijkstra.restype = i32; L.mnb_dijkstra.argtypes = [vp, u32, i64, dbl, dbl, vp, vp]
+    L.mnb_dijkstra_batch.restype = i32; L.mnb_dijkstra_batch.argtypes = [vp, u32, vp, dbl, vp, vp]
     L.mnb_cvp.restype = i32; L.mnb_cvp.argtypes = [vp, u32, vp, i64, dbl, dbl, vp, vp, vp, vp]
     L.mnb_cvp_batch.restype = i32; L.mnb_cvp_batch.argtypes = [vp, u32, vp, vp, dbl, vp]
     L.mnb_inflate.restype = i32; L.mnb_inflate.argtypes = [vp, vp, u32, vp, C.POINTER(InflationParams), vp, vp]

@@ -233,6 +233,12 @@ class MeshMap:
         sp = np.ascontiguousarray(seed_pos, dtype=np.float32).reshape(-1, 3)
         return self._check(self.L.mnb_cvp_batch(self._ctx, sf.size, _p(sf), _p(sp), float(cost_limit), _p(d_out)))
 
+    def dijkstra_batch_dev(self, seed_vertices, cost_limit, d_dist: int, d_pred: int = 0) -> int:
+        """mnb_dijkstra_batch into device rows [n][V] (needs use_device_pointers(True)); d_pred = 0: no predecessors"""
+        sv = np.ascontiguousarray(seed_vertices, dtype=np.uint32).ravel()
+        return self._check(self.L.mnb_dijkstra_batch(self._ctx, sv.size, _p(sv), float(cost_limit), _p(d_dist),
+                                                     _p(d_pred) if d_pred else None))
+
 
 class DijkstraMeshPlanner:
     """dijkstra_mesh_planner::DijkstraMeshPlanner -- wavefront part (dijkstra():217-398)."""
@@ -248,6 +254,16 @@ class DijkstraMeshPlanner:
         pred = np.empty(m.V, dtype=np.uint32)
         rc = m._check(m.L.mnb_dijkstra(m._ctx, int(seed_vertex), int(robot_vertex), float(self.cost_limit),
                                        float(self.goal_dist_offset), _p(dist), _p(pred)))
+        return dict(outcome=rc, dist=dist, pred=pred, **m.stats())
+
+    def dijkstraBatch(self, seed_vertices, want_pred: bool = True):
+        """full-field dijkstra() for many goals in one call (mnb_dijkstra_batch): row k of dist / pred is what
+        dijkstra(seed_vertices[k]) returns; the vector field of goal k is computeVectorMap(pred[k])"""
+        m = self.map
+        sv = np.ascontiguousarray(seed_vertices, dtype=np.uint32).ravel()
+        dist = np.empty((sv.size, m.V), dtype=np.float32)
+        pred = np.empty((sv.size, m.V), dtype=np.uint32) if want_pred else None
+        rc = m._check(m.L.mnb_dijkstra_batch(m._ctx, sv.size, _p(sv), float(self.cost_limit), _p(dist), _p(pred)))
         return dict(outcome=rc, dist=dist, pred=pred, **m.stats())
 
     def computeVectorMap(self, pred):

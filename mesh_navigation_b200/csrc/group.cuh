@@ -33,7 +33,8 @@ struct Nccl {
     return true;
   }
 };
-constexpr int NCCL_FLOAT32 = 7;   // ncclFloat32 (nccl.h: ncclDataType_t)
+constexpr int NCCL_UINT32 = 3;    // ncclUint32  (nccl.h: ncclDataType_t)
+constexpr int NCCL_FLOAT32 = 7;   // ncclFloat32
 }  // namespace mnbg
 
 struct mnb_group {
@@ -41,9 +42,12 @@ struct mnb_group {
   std::vector<mnbg::ncclComm_t> comm;
   std::vector<float*> d_fields;         // per device: [N][pad][V] gathered potentials (library-owned, grows on demand)
   std::vector<size_t> cap;
+  std::vector<uint32_t*> d_preds;       // per device: [N][pad][V] predecessors of the last Dijkstra batch with want_pred
+  std::vector<size_t> pred_cap;
   mnbg::Nccl nccl;
   std::string err;
   uint32_t last_n = 0, last_pad = 0;
+  bool last_has_pred = false;           // the last sharded call was mnb_dijkstra_batch_sharded with want_pred
 };
 
 extern "C" {
@@ -65,6 +69,7 @@ int32_t mnb_group_create(int32_t n_devices, const int32_t* devices, mnb_group** 
   }
   if (rc != MNB_OK) { for (mnb_ctx* c : g->ctx) mnb_destroy(c); delete g; return rc; }
   g->d_fields.assign((size_t)n_devices, nullptr); g->cap.assign((size_t)n_devices, 0);
+  g->d_preds.assign((size_t)n_devices, nullptr); g->pred_cap.assign((size_t)n_devices, 0);
   *out_group = g;
   return MNB_OK;
 }
@@ -74,6 +79,7 @@ void mnb_group_destroy(mnb_group* g) {
   for (size_t r = 0; r < g->ctx.size(); ++r) {
     cudaSetDevice(g->ctx[r]->device);
     if (g->d_fields[r]) cudaFree(g->d_fields[r]);
+    if (g->d_preds[r]) cudaFree(g->d_preds[r]);
     if (r < g->comm.size() && g->comm[r]) g->nccl.CommDestroy(g->comm[r]);
     mnb_destroy(g->ctx[r]);
   }
@@ -113,6 +119,36 @@ int32_t mnb_group_update_vertex_costs(mnb_group* g, uint32_t n_changed, const ui
   });
 }
 
+// grows the per-device [N][pad][V] buffers of a sharded call to hold `need` elements
+extern "C++" {
+template <class T>
+static int32_t group_grow(mnb_group* g, std::vector<T*>& buf, std::vector<size_t>& cap, size_t need) {
+  for (size_t r = 0; r < g->ctx.size(); ++r) {
+    if (cap[r] >= need) continue;
+    cudaSetDevice(g->ctx[r]->device);
+    if (buf[r]) cudaFree(buf[r]);
+    buf[r] = nullptr; cap[r] = 0;
+    if (cudaMalloc((void**)&buf[r], need * sizeof(T)) != cudaSuccess) { g->err = "gather buffer: out of device memory"; return MNB_E_NOMEM; }
+    cap[r] = need;
+  }
+  return MNB_OK;
+}
+}  // extern "C++"
+
+// in-place all-gather of every rank's slot of the fields (and, with preds, of the predecessors) in one NCCL group call
+static int32_t group_gather(mnb_group* g, size_t slot, bool preds) {
+  const size_t N = g->ctx.size();
+  if (g->nccl.GroupStart() != 0) { g->err = "ncclGroupStart"; return MNB_E_NCCL; }
+  for (size_t r = 0; r < N; ++r) {
+    int e = g->nccl.AllGather(g->d_fields[r] + r * slot, g->d_fields[r], slot, mnbg::NCCL_FLOAT32, g->comm[r], g->ctx[r]->stream);
+    if (e == 0 && preds) e = g->nccl.AllGather(g->d_preds[r] + r * slot, g->d_preds[r], slot, mnbg::NCCL_UINT32, g->comm[r], g->ctx[r]->stream);
+    if (e != 0) { g->nccl.GroupEnd(); g->err = std::string("ncclAllGather: ") + (g->nccl.GetErrorString ? g->nccl.GetErrorString(e) : "?"); return MNB_E_NCCL; }
+  }
+  if (g->nccl.GroupEnd() != 0) { g->err = "ncclGroupEnd"; return MNB_E_NCCL; }
+  for (size_t r = 0; r < N; ++r) { cudaSetDevice(g->ctx[r]->device); if (cudaStreamSynchronize(g->ctx[r]->stream) != cudaSuccess) { g->err = "gather: stream sync failed"; return MNB_E_CUDA; } }
+  return MNB_OK;
+}
+
 // Batched full-field CVP plans, sharded: goal k -> rank k mod N.  Every rank plans its goals (mnb_cvp_batch on its device,
 // all devices concurrently) straight into its slot of the gather buffer; one in-place ncclAllGather then leaves ALL fields
 // on EVERY device.  Layout of the per-device result (library-owned device memory, valid until the next sharded call):
@@ -123,16 +159,10 @@ int32_t mnb_cvp_batch_sharded(mnb_group* g, uint32_t n, const uint32_t* seed_fac
   const uint32_t N = (uint32_t)g->ctx.size(), pad = (n + N - 1) / N;
   const size_t V = g->ctx[0]->V;
   if (!V) { g->err = "mnb_group_set_mesh / mnb_group_set_costs not called"; return MNB_E_STATE; }
-  const size_t need = (size_t)N * pad * V;
-  for (size_t r = 0; r < N; ++r) {
-    if (g->cap[r] >= need) continue;
-    cudaSetDevice(g->ctx[r]->device);
-    if (g->d_fields[r]) cudaFree(g->d_fields[r]);
-    g->d_fields[r] = nullptr; g->cap[r] = 0;
-    if (cudaMalloc((void**)&g->d_fields[r], need * sizeof(float)) != cudaSuccess) { g->err = "gather buffer: out of device memory"; return MNB_E_NOMEM; }
-    g->cap[r] = need;
-  }
-  const int32_t rc = group_foreach(g, [&](mnb_ctx* c, size_t r) -> int32_t {
+  g->last_has_pred = false;
+  int32_t rc = group_grow(g, g->d_fields, g->cap, (size_t)N * pad * V);
+  if (rc != MNB_OK) return rc;
+  rc = group_foreach(g, [&](mnb_ctx* c, size_t r) -> int32_t {
     std::vector<uint32_t> sf; std::vector<float> sp;
     for (uint32_t k = (uint32_t)r; k < n; k += N) { sf.push_back(seed_faces[k]); sp.insert(sp.end(), seed_pos + 3 * (size_t)k, seed_pos + 3 * (size_t)k + 3); }
     if (sf.empty()) return MNB_OK;
@@ -144,15 +174,35 @@ int32_t mnb_cvp_batch_sharded(mnb_group* g, uint32_t n, const uint32_t* seed_fac
   });
   if (rc != MNB_OK) return rc;
   g->last_n = n; g->last_pad = pad;
-  if (gather && N > 1) {
-    if (g->nccl.GroupStart() != 0) { g->err = "ncclGroupStart"; return MNB_E_NCCL; }
-    for (size_t r = 0; r < N; ++r) {
-      const int e = g->nccl.AllGather(g->d_fields[r] + r * (size_t)pad * V, g->d_fields[r], (size_t)pad * V, mnbg::NCCL_FLOAT32, g->comm[r], g->ctx[r]->stream);
-      if (e != 0) { g->nccl.GroupEnd(); g->err = std::string("ncclAllGather: ") + (g->nccl.GetErrorString ? g->nccl.GetErrorString(e) : "?"); return MNB_E_NCCL; }
-    }
-    if (g->nccl.GroupEnd() != 0) { g->err = "ncclGroupEnd"; return MNB_E_NCCL; }
-    for (size_t r = 0; r < N; ++r) { cudaSetDevice(g->ctx[r]->device); if (cudaStreamSynchronize(g->ctx[r]->stream) != cudaSuccess) { g->err = "gather: stream sync failed"; return MNB_E_CUDA; } }
-  }
+  if (gather && N > 1 && (rc = group_gather(g, (size_t)pad * V, false)) != MNB_OK) return rc;
+  return MNB_SUCCESS;
+}
+
+// Batched full-field Dijkstra plans, sharded the same way (mnb_dijkstra_batch per rank): distances into the fields buffers
+// above, with want_pred the predecessors into d_preds in the same layout; both are gathered in one NCCL group call.
+int32_t mnb_dijkstra_batch_sharded(mnb_group* g, uint32_t n, const uint32_t* seed_vertices, double cost_limit, int32_t want_pred, int32_t gather) {
+  if (!g || n == 0 || !seed_vertices) return MNB_E_ARG;
+  const uint32_t N = (uint32_t)g->ctx.size(), pad = (n + N - 1) / N;
+  const size_t V = g->ctx[0]->V;
+  if (!V) { g->err = "mnb_group_set_mesh / mnb_group_set_costs not called"; return MNB_E_STATE; }
+  g->last_has_pred = false;
+  int32_t rc = group_grow(g, g->d_fields, g->cap, (size_t)N * pad * V);
+  if (rc == MNB_OK && want_pred) rc = group_grow(g, g->d_preds, g->pred_cap, (size_t)N * pad * V);
+  if (rc != MNB_OK) return rc;
+  rc = group_foreach(g, [&](mnb_ctx* c, size_t r) -> int32_t {
+    std::vector<uint32_t> sv;
+    for (uint32_t k = (uint32_t)r; k < n; k += N) sv.push_back(seed_vertices[k]);
+    if (sv.empty()) return MNB_OK;
+    const int old_mode = c->ptr_mode;
+    c->ptr_mode = MNB_PTR_DEVICE;        // (only the outputs are device pointers: seeds are always host arrays)
+    const size_t off = r * (size_t)pad * V;
+    const int32_t b = mnb_dijkstra_batch(c, (uint32_t)sv.size(), sv.data(), cost_limit, g->d_fields[r] + off, want_pred ? g->d_preds[r] + off : nullptr);
+    c->ptr_mode = old_mode;
+    return b;
+  });
+  if (rc != MNB_OK) return rc;
+  g->last_n = n; g->last_pad = pad; g->last_has_pred = want_pred != 0;
+  if (gather && N > 1 && (rc = group_gather(g, (size_t)pad * V, want_pred != 0)) != MNB_OK) return rc;
   return MNB_SUCCESS;
 }
 
@@ -167,6 +217,20 @@ int32_t mnb_group_read_fields(mnb_group* g, int32_t rank, uint32_t first, uint32
   if (cudaSetDevice(c->device) != cudaSuccess) return MNB_E_CUDA;
   for (uint32_t k = 0; k < count; ++k)
     if (cudaMemcpyAsync(out_host + (size_t)k * V, g->d_fields[(size_t)rank] + (size_t)mnb_group_row(g, first + k) * V, sizeof(float) * V, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return MNB_E_CUDA;
+  return cudaStreamSynchronize(c->stream) == cudaSuccess ? MNB_OK : MNB_E_CUDA;
+}
+
+// device pointer of the predecessors on `rank` (uint32[N][pad][V], see mnb_dijkstra_batch_sharded)
+uint32_t* mnb_group_preds(mnb_group* g, int32_t rank) { return (g && rank >= 0 && (size_t)rank < g->ctx.size()) ? g->d_preds[(size_t)rank] : nullptr; }
+// copies the predecessors of goals [first, first + count) from `rank`'s buffer into host memory, in goal order
+int32_t mnb_group_read_preds(mnb_group* g, int32_t rank, uint32_t first, uint32_t count, uint32_t* out_host) {
+  if (!g || rank < 0 || (size_t)rank >= g->ctx.size() || !out_host || first + count > g->last_n) return MNB_E_ARG;
+  if (!g->last_has_pred) { g->err = "mnb_group_read_preds needs a preceding mnb_dijkstra_batch_sharded with want_pred"; return MNB_E_STATE; }
+  mnb_ctx* c = g->ctx[(size_t)rank];
+  const size_t V = c->V;
+  if (cudaSetDevice(c->device) != cudaSuccess) return MNB_E_CUDA;
+  for (uint32_t k = 0; k < count; ++k)
+    if (cudaMemcpyAsync(out_host + (size_t)k * V, g->d_preds[(size_t)rank] + (size_t)mnb_group_row(g, first + k) * V, sizeof(uint32_t) * V, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return MNB_E_CUDA;
   return cudaStreamSynchronize(c->stream) == cudaSuccess ? MNB_OK : MNB_E_CUDA;
 }
 

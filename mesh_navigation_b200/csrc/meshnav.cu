@@ -21,6 +21,7 @@ using namespace mnb;
 #include "launch.cuh"
 #include "kernels_maps.cuh"
 #include "kernels_wavefront.cuh"
+#include "dijkstra_batch.cuh"
 #include "kernels_layers.cuh"
 #include "kernels_field.cuh"
 #include "kernels_updates.cuh"
@@ -64,6 +65,10 @@ struct mnb_ctx {
   const uint32_t* last_pred = nullptr; const float* last_dir = nullptr; const int32_t* last_cut = nullptr;
   uint32_t last_seed_face = 0; float last_seed_pos[3] = {0, 0, 0}; bool last_valid = false;
   float* d_path_pos = nullptr; uint32_t* d_path_face = nullptr; int32_t* d_bt_result = nullptr; uint32_t path_cap = 0;
+  // scratch of mnb_dijkstra_batch (dijkstra_batch.cuh): its own, so that a batch leaves the wavefront workspace and the
+  // device-resident result of the last mnb_cvp alone
+  uint32_t* d_djb_scratch = nullptr; GroupCtl* d_djb_ctl = nullptr; uint32_t djb_groups = 0;
+  uint32_t* d_djb_seeds = nullptr; uint32_t djb_seed_cap = 0; uint32_t* d_djb_pred = nullptr; size_t djb_pred_cap = 0;
   uint32_t* d_lethals = nullptr; uint32_t lethal_cap = 0; uint8_t* d_infl_invalid = nullptr; float* d_out_cost = nullptr;
   // repulsive vector field of the last inflation (InflationLayer::vector_map_ / distances_)
   bool infl_labels_valid = false, infl_had_invalid = false, infl_field_valid = false, repulsive_on = false;
@@ -133,6 +138,7 @@ static void free_mesh(mnb_ctx* c) {
   c->infl_labels_valid = false; c->infl_field_valid = false; c->repulsive_on = false;
   dfree(c->d_prev_risk); c->prev_risk_valid = false; dfree(c->d_upd_ids); dfree(c->d_upd_costs); c->upd_cap = 0; c->upd_cost_cap = 0; dfree(c->d_upd_stamp); c->upd_call = 0;
   dfree(c->d_changed); dfree(c->d_tile_count); dfree(c->d_total);
+  dfree(c->d_djb_scratch); dfree(c->d_djb_ctl); c->djb_groups = 0; dfree(c->d_djb_pred); c->djb_pred_cap = 0;
   dfree(c->d_path_pos); dfree(c->d_path_face); dfree(c->d_bt_result); c->path_cap = 0; c->last_valid = false;
   dfree(c->d_face_normals); dfree(c->d_vertex_normals); dfree(c->d_border); dfree(c->d_layer_costs); dfree(c->d_layer_combined);
   dfree(c->d_layer_mask); dfree(c->d_clearance); dfree(c->d_overflow); dfree(c->d_pos4); dfree(c->d_vn4); dfree(c->d_nbr8);
@@ -208,7 +214,7 @@ void mnb_destroy(mnb_ctx* ctx) {
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
   free_mesh(ctx);
-  dfree(ctx->d_next_query); dfree(ctx->d_seed_faces); dfree(ctx->d_seed_pos); dfree(ctx->d_lethals);
+  dfree(ctx->d_next_query); dfree(ctx->d_seed_faces); dfree(ctx->d_seed_pos); dfree(ctx->d_lethals); dfree(ctx->d_djb_seeds);
   if (ctx->h_cancel) cudaFreeHost(ctx->h_cancel);
   if (ctx->ev0) cudaEventDestroy(ctx->ev0);
   if (ctx->ev1) cudaEventDestroy(ctx->ev1);
@@ -539,9 +545,9 @@ static int32_t launch_cvp(mnb_ctx* ctx, const CvpKernelArgs& a, int cs, unsigned
   return MNB_OK;
 }
 
-static int32_t finish_stats(mnb_ctx* ctx, unsigned groups, unsigned launches) {
+static int32_t finish_stats(mnb_ctx* ctx, unsigned groups, unsigned launches, const GroupCtl* ctl = nullptr) {
   std::vector<GroupCtl> h(groups);
-  CK(cudaMemcpyAsync(h.data(), ctx->ws.ctl, sizeof(GroupCtl) * groups, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(h.data(), ctl ? ctl : ctx->ws.ctl, sizeof(GroupCtl) * groups, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   ctx->stats.rounds = 0; ctx->stats.recomputes = 0; ctx->stats.settled = 0;
   ctx->stats.skipped = 0; ctx->stats.deep_labels = 0; ctx->stats.pool_words = 0;
@@ -781,6 +787,68 @@ static int32_t impl_dijkstra(mnb_ctx* ctx, uint32_t seed_vertex, int64_t robot_v
   if ((rc = finish_stats(ctx, 1, 1)) != MNB_OK) return rc;
   if (ctx->h_cancel && *ctx->h_cancel) return MNB_CANCELED;
   if (robot_vertex >= 0 && rp == (uint32_t)robot_vertex) return MNB_NO_PATH_FOUND;          // dijkstra:358-362
+  return MNB_SUCCESS;
+}
+
+static int32_t impl_dijkstra_batch(mnb_ctx* ctx, uint32_t n, const uint32_t* seed_vertices, double cost_limit, float* out_dist,
+                                   uint32_t* out_pred) {
+  if (!ctx || !seed_vertices || !out_dist || !ctx->V || n == 0) return MNB_E_ARG;
+  if (!ctx->costs_set) { ctx->err = "costs not set"; return MNB_E_STATE; }
+  for (uint32_t i = 0; i < n; ++i) if (seed_vertices[i] >= ctx->V) return MNB_INVALID_START;
+  CK(cudaSetDevice(ctx->device));
+  int per_sm = 1;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_dijkstra_batch<1>, DJB_THREADS, 0));
+  per_sm = std::max(1, std::min(per_sm, (int)DJB_MINBLOCKS));
+  const unsigned slots = (unsigned)(ctx->sm_count * per_sm);
+  // CTAs per goal as in impl_cvp_batch: one when the goals fill the machine, a cluster when there are fewer goals than slots
+  int cs = ctx->batch_cluster;
+  if (cs <= 0) { cs = 1; while (cs < 8 && (unsigned)(2 * cs) * n <= slots) cs *= 2; }
+  unsigned groups = std::max(1u, std::min(slots / (unsigned)cs, n));
+  const size_t V = ctx->V;
+  if (groups > ctx->djb_groups) {
+    dfree(ctx->d_djb_scratch); dfree(ctx->d_djb_ctl); ctx->djb_groups = 0;
+    CK(dalloc(&ctx->d_djb_scratch, (size_t)groups * 3 * V)); CK(dalloc(&ctx->d_djb_ctl, (size_t)groups));
+    ctx->djb_groups = groups;
+  }
+  if (n > ctx->djb_seed_cap) { dfree(ctx->d_djb_seeds); ctx->djb_seed_cap = 0; CK(dalloc(&ctx->d_djb_seeds, (size_t)n)); ctx->djb_seed_cap = n; }
+  const bool dev = ctx->ptr_mode == MNB_PTR_DEVICE;
+  int32_t rc;
+  if (!dev) {
+    if ((rc = ensure_out(ctx, (size_t)n * V, false)) != MNB_OK) return rc;
+    if (out_pred && (size_t)n * V > ctx->djb_pred_cap) {
+      dfree(ctx->d_djb_pred); ctx->djb_pred_cap = 0; CK(dalloc(&ctx->d_djb_pred, (size_t)n * V)); ctx->djb_pred_cap = (size_t)n * V;
+    }
+  }
+  if ((rc = ensure_adj_tables(ctx)) != MNB_OK) return rc;
+  if (ctx->h_cancel) *ctx->h_cancel = 0;
+  CK(cudaMemcpyAsync(ctx->d_djb_seeds, seed_vertices, sizeof(uint32_t) * n, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemsetAsync(ctx->d_next_query, 0, sizeof(unsigned int), ctx->stream));
+  CK(cudaMemsetAsync(ctx->d_djb_ctl, 0, sizeof(GroupCtl) * groups, ctx->stream));
+  DijkstraBatchArgs a{};
+  a.V = ctx->V; a.adj_ptr = ctx->d_adj_ptr; a.adj_nw = ctx->d_adj_nw; a.ell_adj = ctx->d_ell_adj;
+  a.cost = ctx->d_cost; a.invalid = ctx->has_invalid ? ctx->d_invalid : nullptr; a.cost_limit = cost_limit;
+  a.delta = ctx->delta; a.n_queries = n; a.seeds = ctx->d_djb_seeds;
+  a.out_dist = dev ? out_dist : ctx->d_out_dist;
+  a.out_pred = !out_pred ? nullptr : (dev ? out_pred : ctx->d_djb_pred);
+  a.scratch = ctx->d_djb_scratch; a.ctl = ctx->d_djb_ctl; a.next_query = ctx->d_next_query; a.cancel_flag = ctx->d_cancel;
+  a.max_rounds = watchdog_rounds(ctx->V);
+  CK(cudaEventRecord(ctx->ev0, ctx->stream));
+  cudaError_t e;
+  const unsigned blocks = groups * (unsigned)cs;
+  switch (cs) {
+    case 1: e = launch_cluster(k_dijkstra_batch<1>, a, 1, blocks, DJB_THREADS, ctx->stream); break;
+    case 2: e = launch_cluster(k_dijkstra_batch<2>, a, 2, blocks, DJB_THREADS, ctx->stream); break;
+    case 4: e = launch_cluster(k_dijkstra_batch<4>, a, 4, blocks, DJB_THREADS, ctx->stream); break;
+    default: e = launch_cluster(k_dijkstra_batch<8>, a, 8, blocks, DJB_THREADS, ctx->stream); break;
+  }
+  if (e != cudaSuccess) { ctx->err = std::string("dijkstra batch launch: ") + cudaGetErrorString(e); return MNB_E_CUDA; }
+  CK(cudaEventRecord(ctx->ev1, ctx->stream));
+  if (!dev) {
+    CK(cudaMemcpyAsync(out_dist, a.out_dist, sizeof(float) * (size_t)n * V, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out_pred) CK(cudaMemcpyAsync(out_pred, a.out_pred, sizeof(uint32_t) * (size_t)n * V, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  if ((rc = finish_stats(ctx, groups, 1, ctx->d_djb_ctl)) != MNB_OK) return rc;
+  if (ctx->h_cancel && *ctx->h_cancel) return MNB_CANCELED;
   return MNB_SUCCESS;
 }
 
@@ -1231,6 +1299,9 @@ int32_t mnb_cvp_batch(mnb_ctx* ctx, uint32_t n, const uint32_t* seed_faces, cons
 int32_t mnb_dijkstra(mnb_ctx* ctx, uint32_t seed_vertex, int64_t robot_vertex, double cost_limit, double goal_dist_offset,
                      float* out_dist, uint32_t* out_pred) {
   return guarded(ctx, [&]() { return impl_dijkstra(ctx, seed_vertex, robot_vertex, cost_limit, goal_dist_offset, out_dist, out_pred); });
+}
+int32_t mnb_dijkstra_batch(mnb_ctx* ctx, uint32_t n, const uint32_t* seed_vertices, double cost_limit, float* out_dist, uint32_t* out_pred) {
+  return guarded(ctx, [&]() { return impl_dijkstra_batch(ctx, n, seed_vertices, cost_limit, out_dist, out_pred); });
 }
 int32_t mnb_inflate(mnb_ctx* ctx, const uint32_t* lethals, uint32_t n, const uint8_t* invalid,
                     const mnb_inflation_params* params, float* out_dist, float* out_cost) {
